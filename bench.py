@@ -2,8 +2,11 @@
 """bench.py -- persons/s of the simple-HRNet hot path (network forward + argmax decode) on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-cuda]
-                  [--config w48|w32|poseresnet50]
+                  [--config w48|w32|poseresnet50] [--dump-outputs DIR]
   (N > 1: launched by torchrun, one rank per GPU; crops sharded by batch, one NCCL all-gather of joints)
+  --dump-outputs DIR: after the timed steps, the joints [B,17,3] (y, x, confidence) the last timed step returned are
+  written to DIR/joints.npy (float32).  Weights and inputs are seeded, so two builds run with the same arguments can be
+  compared output for output.
 
 One "step" = one pass of the hot path over one batch of synthetic crops.  Default config = BASELINE.json configs[2],
 the one the metric is quoted on: HRNet-W48 @ 384x288, 17 joints, 64 persons per GPU, random-init weights
@@ -33,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is written or cached there
 
 J = 17
 CONFIGS = {
@@ -331,7 +335,10 @@ def main():
     ap.add_argument("--no-kernel-roofline", action="store_true")
     ap.add_argument("--flags", type=int, default=0, help="HRNET_FLAG_* plan flags (experiments)")
     ap.add_argument("--tune", default="", help="HRNET_TUNE_* overrides, e.g. 0=400,1=250 (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the joints of the last timed step to DIR/joints.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
     cfg = CONFIGS[args.config]
 
@@ -348,10 +355,11 @@ def main():
     import numpy as np
     import torch
     import torch.distributed as dist
-    from simple_hrnet_b200 import B200Engine, HostPipeline, ShardedPredictor, shard_range
+    from simple_hrnet_b200 import B200Engine, HostPipeline, ShardedPredictor, load_library, shard_range
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (the product path has no CPU fallback)")
+    load_library(build_if_missing=False)     # the library build() made; bench never compiles into the tree
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     if world > 1:
@@ -420,6 +428,9 @@ def main():
     ms_total = float(ms.item())
     clocks = sampler.stop() if rank == 0 else None
     value = B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "joints.npy"), joints.cpu().numpy().astype(np.float32))
 
     # ---- multi-GPU correctness of the gathered result (outside the timed region): every rank recomputes the shard of
     # rank (r+1) % world from that rank's seed and compares it bit for bit with its slice of the gathered joints

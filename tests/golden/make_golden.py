@@ -131,8 +131,66 @@ def decode_fixture():
     print("decode_edge: ok", boxes[0])
 
 
+STATE_DICT_CONFIGS = [("hrnet", 32), ("hrnet", 48), ("poseresnet", 50), ("poseresnet", 101)]
+
+
+def state_dict_fixture():
+    """Key set, shapes and dtypes of the reference modules' state_dicts (the layout of the official pose_hrnet_* /
+    pose_resnet_* checkpoints), in the modules' own order."""
+    from models_.hrnet import HRNet
+    from models_.poseresnet import PoseResNet
+    out = {}
+    for arch, c in STATE_DICT_CONFIGS:
+        sd = (HRNet(c, 17) if arch == "hrnet" else PoseResNet(c, 17)).state_dict()
+        tag = f"{arch}{c}"
+        out[tag + "_keys"] = np.asarray(list(sd.keys()))
+        out[tag + "_ndim"] = np.asarray([t.dim() for t in sd.values()], dtype=np.int32)
+        out[tag + "_dims"] = np.asarray([d for t in sd.values() for d in t.shape], dtype=np.int32)
+        out[tag + "_dtypes"] = np.asarray([str(t.dtype).replace("torch.", "") for t in sd.values()])
+        print(f"reference_state_dicts: {tag} {len(sd)} keys")
+    np.savez_compressed(os.path.join(HERE, "reference_state_dicts.npz"), **out)
+
+
+SEAM_CASES = [("hrnet", 32, (256, 192), 6), ("hrnet", 48, (384, 288), 5), ("poseresnet", 50, (256, 192), 3)]
+SEAM_SAMPLE = 2048
+
+
+def seam_fixture():
+    """The reference's SimpleHRNet(device=cpu, max_batch_size=4).predict on one image at another resolution (it is resized)
+    and on a stack longer than max_batch_size (it is chunked).  Heat-maps are too large to store whole: a fixed sample of
+    SEAM_SAMPLE values per input, max |heat-map| and the top-1 / top-2 gaps are kept, boxes and joints in full."""
+    from SimpleHRNet import SimpleHRNet
+    out = {}
+    for arch, c, res, batch in SEAM_CASES:
+        spec = O.hrnet_param_spec(c, 17) if arch == "hrnet" else O.poseresnet_param_spec(c, 17)
+        sd = O.make_state_dict(spec, seed=0, bn="default")
+        with tempfile.TemporaryDirectory() as td:
+            ck = os.path.join(td, "w.pth")
+            torch.save(sd, ck)
+            m = SimpleHRNet(c, 17, ck, model_name="HRNet" if arch == "hrnet" else "PoseResNet", resolution=res,
+                            multiperson=False, return_heatmaps=True, return_bounding_boxes=True, max_batch_size=4,
+                            device=torch.device("cpu"))
+        rng = np.random.default_rng(7)
+        img = rng.integers(0, 256, (300, 210, 3), dtype=np.uint8)
+        stack = rng.integers(0, 256, (batch, res[0], res[1], 3), dtype=np.uint8)
+        for kind, inp in (("img", img), ("stack", stack)):
+            hm, boxes, pts = m.predict(inp)
+            ohm, oboxes, opts = O.predict(sd, inp, res, model=arch, resnet_size=c)
+            assert np.array_equal(hm, ohm) and np.array_equal(boxes, oboxes) and np.array_equal(pts, opts), \
+                f"{arch}{c} {kind}: oracle predict != reference predict"
+            tag = f"{arch}{c}_{kind}"
+            at = np.sort(np.random.default_rng(0).choice(hm.size, SEAM_SAMPLE, replace=False)).astype(np.int64)
+            out.update({tag + "_hm_shape": np.asarray(hm.shape), tag + "_hm_at": at, tag + "_hm_values": hm.ravel()[at],
+                        tag + "_hm_absmax": np.float32(np.abs(hm).max()), tag + "_gaps": gaps(hm),
+                        tag + "_boxes": boxes, tag + "_pts": pts})
+            print(f"reference_seam_predict: {tag} hm {hm.shape} max|hm| {np.abs(hm).max():.4f} pts {pts.shape}")
+    np.savez_compressed(os.path.join(HERE, "reference_seam_predict.npz"), **out)
+
+
 if __name__ == "__main__":
-    torch.set_num_threads(os.cpu_count())
+    torch.set_num_threads(8)             # tests/test_oracle.py replays the fixtures bit for bit with the same count
+    state_dict_fixture()
+    seam_fixture()
     decode_fixture()
     # tiny net-level fixture for fast CPU tests (resolution must be a multiple of 32)
     model_fixture("w32_64x64_n2_rand", "hrnet", 32, 2, 64, 64, wseed=3, bn="random", xseed=5)
